@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: Mpixels/s of REBLUR_DIFFUSE_SPECULAR at 3840x2160 (BASELINE.json metric), one frame per step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--width 3840 --height 2160]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--width 3840 --height 2160] [--dump-outputs DIR]
+
+Runs on the tree as `python -m raytracingdenoiser_b200.build` left it and writes nothing there.
 
 value     whole chain, inputs already resident in HBM (each frame's inputs are separate 265 MB buffers, i.e. larger than
           the 126 MB L2, so no flush is needed between steps), CUDA events on the launching stream, max over ranks.
@@ -15,6 +17,10 @@ roofline  Blur + PostBlur (the north-star kernels): algorithmic bytes (92 B/px, 
           rank 0 include the wait for the slowest peer.
 cpu_baseline / --impl reference   the CPU restatement of the reference shaders (oracle/, OpenMP over all host cores) on a
           bounded sample of the same frames.  It is a reported baseline; the oracle is never on the product path.
+--dump-outputs DIR   after the timed steps, the outputs of the last timed step (OUT_DIFF_RADIANCE_HITDIST, OUT_SPEC_RADIANCE_HITDIST
+          as float32) go to DIR/<name>.npy: whole (height, width, 4) arrays when all of them fit into 64 MB, otherwise the same fixed,
+          seeded sample of texels of each, (texels, 4).  The inputs depend only on the arguments, so two builds can be compared
+          output for output.  One GPU only.
 """
 import argparse
 import json
@@ -148,6 +154,27 @@ def run_cpu_reference(width, height, frames, steps, warmup):
     return width * height * len(times) / total / 1e6, 1e3 * total / len(times), info
 
 
+DUMP_BYTES = 64 * 1000 * 1000  # all files together, .npy headers included
+
+
+def dump_outputs(directory, outputs):
+    """Writes {name: (H, W, C) tensor} as float32 DIR/<name>.npy: whole when everything fits into DUMP_BYTES, otherwise the texels
+    of one fixed, seeded sample (the same texels for every output, in raster order)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    arrays = {n: t.float().cpu().numpy() for n, t in outputs.items()}
+    data_bytes = DUMP_BYTES - 1024 * len(arrays)
+    sample = None
+    if sum(a.size * 4 for a in arrays.values()) > data_bytes:
+        h, w = next(iter(arrays.values())).shape[:2]
+        texels = data_bytes // sum(a[0, 0].size * 4 for a in arrays.values())
+        sample = np.sort(np.random.default_rng(20240917).choice(h * w, size=texels, replace=False))
+    for n, a in arrays.items():
+        if sample is not None:
+            a = a.reshape((a.shape[0] * a.shape[1],) + a.shape[2:])[sample]
+        np.save(os.path.join(directory, n + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -157,12 +184,15 @@ def main():
     ap.add_argument("--width", type=int, default=3840)
     ap.add_argument("--height", type=int, default=2160)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1:
+        ap.error("--dump-outputs needs --gpus 1")
 
     import torch
-    from raytracingdenoiser_b200 import build
-    build.build_all()
-    from raytracingdenoiser_b200 import harness, nrd
+    from raytracingdenoiser_b200 import harness, nrd  # nrd raises if the library is not built
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -290,6 +320,8 @@ def main():
         gpu.denoise(harness.make_common_settings(frames[i], W, H, i))
     e1.record(stream)
     barrier()
+    if args.dump_outputs:  # before the per-pass and end-to-end runs below denoise further frames into the same textures
+        dump_outputs(args.dump_outputs, gpu.outputs())
     launches = nrd.launch_count() - l0
     ms_total = e0.elapsed_time(e1)
     if world > 1:

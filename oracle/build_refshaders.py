@@ -67,8 +67,9 @@ def fix_hlsl(text):
     text = IN_PARAM.sub(r"\1", text)
     text = FLOAT_LITERAL.sub(r"\1f", text)
     text = re.sub(r"\bgroupshared\b", "static", text)
-    # a vector initialised from a one-channel texture fetch (HLSL replicates the scalar): float2 data = gIn_Penumbra[ pixelPos ];
-    text = re.sub(r"\b(float[234])\s+(\w+)\s*=\s*(gIn_\w+\s*\[[^\]]*\])\s*;", r"\1 \2 = \1(float(\3));", text)
+    # a vector initialised from a texture fetch: HLSL replicates a one-channel fetch (float2 data = gIn_Penumbra[ pixelPos ];),
+    # a vector fetch is taken as it is (hlsl_cpp.h _fetch_init)
+    text = re.sub(r"\b(float[234])\s+(\w+)\s*=\s*(gIn_\w+\s*\[[^\]]*\])\s*;", r"\1 \2 = _fetch_init<\1>(\3);", text)
     # x.xxx on a scalar (HLSL: float3(x)) -- also harmless on a vector
     text = re.sub(r"((?<![\w.])\d[\d.]*(?:[eE][-+]?\d+)?f)\s*\.(x{2,4})\b", r"_splat_\2(\1)", text)
     text = re.sub(r"(?<![\w.\])])([A-Za-z_]\w*)\.(x{2,4})\b", r"_splat_\2(\1)", text)

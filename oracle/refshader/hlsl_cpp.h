@@ -204,6 +204,10 @@ struct float1
     explicit float1(float v) : x(v) {}
     operator float() const { return x; }
 };
+// floatN x = gIn_T[ p ]; build_refshaders.py rewrites the initialiser into _fetch_init<floatN>( gIn_T[ p ] ): a one-channel fetch
+// (float1) is replicated like HLSL does, a vector fetch initialises the vector as it is
+template <class V> inline V _fetch_init(const float1& a) { return V(float(a)); }
+template <class V, class T> inline V _fetch_init(const T& a) { return V(a); }
 template <class T> struct TexelOf;
 struct TexelGatherFloat
 {

@@ -5,6 +5,9 @@ asks for (as numpy arrays), binds resources in DispatchDesc order and runs each 
 Only tests/, __graft_entry__.smoke() and bench.py's CPU legs may import this.
 """
 import ctypes as C
+import hashlib
+import io
+import lzma
 import os
 
 import numpy as np
@@ -72,15 +75,83 @@ _NP = {nrd.Format.R8_UNORM: (np.uint8, 1), nrd.Format.R8_UINT: (np.uint8, 1), nr
 
 _REFSHADERS = {}
 
+# The reference's pass shaders compiled for the CPU (oracle/_ref/shaders, built only where the reference sources are present) are
+# not part of the repository.  What the tests need of them is recorded in tests/golden/reference_shader_outputs.npz.xz by
+# tests/golden/make_reference_golden.py: for every dispatch the tests run, keyed by a hash of its input state (shader,
+# constants, grid, rect origin, every bound texture), the texels where the shader's outputs differ from the oracle's and a hash of
+# each output.  run_reference_shader() replays a record: it runs the oracle's pass, writes the recorded texels over it and checks the
+# result against the recorded hash, so the tests see the shader's exact output.  A dispatch that was not recorded, or an oracle
+# whose output has changed since the recording, is an error, not a silent fall-back.
+REFERENCE_GOLDEN = os.path.join(_ROOT, "tests", "golden", "reference_shader_outputs.npz.xz")  # (an .npz, xz-compressed)
+RECORD_ENV = "NRD_B200_RECORD_REFERENCE_SHADERS"  # "1": run the compiled shaders and record them (make_reference_golden.py)
+_recorded = {}
+_golden = {}
+
+
+def _recording():
+    return os.environ.get(RECORD_ENV) == "1"
+
+
+def _golden_records():
+    if not _golden:
+        with lzma.open(REFERENCE_GOLDEN) as f:
+            z = np.load(io.BytesIO(f.read()))
+        _golden["shaders"] = set(str(s) for s in z["shaders"])
+        _golden["index"] = {bytes(k): i for i, k in enumerate(z["keys"])}
+        for k in ("out_start", "out_sha", "diff_start", "diff_index", "value_start", "diff_value"):
+            _golden[k] = z[k]
+    return _golden
+
+
+def _shader_name(shader_file_name):
+    return shader_file_name[:-3] if shader_file_name.endswith(".cs") else shader_file_name
+
+
+def has_reference_shader(shader_file_name):
+    """Whether the reference has a compiled pass shader for this dispatch (the Clear_* passes have none)."""
+    if _recording():
+        return os.path.exists(reference_shader_path(shader_file_name))
+    return _shader_name(shader_file_name) in _golden_records()["shaders"]
+
+
+def _texels(arr):
+    """(texels, bytes per texel) uint8 view of a texture (writes go through to it)."""
+    return arr.reshape(arr.shape[0] * arr.shape[1], -1).view(np.uint8)
+
+
+def _digest(arr):
+    return hashlib.sha1(np.ascontiguousarray(arr).tobytes()).digest()[:8]
+
+
+def save_reference_recording(path=REFERENCE_GOLDEN):
+    """Writes what run_reference_shader() recorded (in RECORD_ENV mode) to `path`."""
+    keys = sorted(_recorded)
+    out_start, out_sha, diff_start, value_start, diff_index, diff_value = [0], [], [0], [0], [], []
+    for k in keys:
+        for sha, idx, val in _recorded[k]:
+            out_sha.append(np.frombuffer(sha, dtype=np.uint8))
+            diff_index.append(np.diff(idx, prepend=0))  # (gaps compress better than positions)
+            diff_value.append(val.T.reshape(-1))         # byte planes: the XOR of nearly equal values is zero in its high bytes
+            diff_start.append(diff_start[-1] + len(idx))
+            value_start.append(value_start[-1] + val.size)
+        out_start.append(len(out_sha))
+    built = sorted(f[:-3] for f in os.listdir(os.path.dirname(reference_shader_path("x"))) if f.endswith(".so"))
+    buf = io.BytesIO()
+    np.savez(buf, keys=np.array([np.frombuffer(k, dtype=np.uint8) for k in keys]).reshape(-1, 8), shaders=np.array(built),
+             out_start=np.array(out_start, dtype=np.int32), out_sha=np.array(out_sha).reshape(-1, 8),
+             diff_start=np.array(diff_start, dtype=np.int64), value_start=np.array(value_start, dtype=np.int64),
+             diff_index=np.concatenate(diff_index).astype(np.int32), diff_value=np.concatenate(diff_value).astype(np.uint8))
+    with lzma.open(path, "wb", preset=9 | lzma.PRESET_EXTREME) as f:
+        f.write(buf.getvalue())
+
 
 def reference_shader_path(shader_file_name):
-    name = shader_file_name[:-3] if shader_file_name.endswith(".cs") else shader_file_name
-    return os.path.join(_ROOT, "oracle", "_ref", "shaders", name + ".so")
+    return os.path.join(_ROOT, "oracle", "_ref", "shaders", _shader_name(shader_file_name) + ".so")
 
 
 def reference_shader_lib(shader_file_name):
-    """The reference's own shader source of one pass, compiled for the CPU by oracle/build_refshaders.py (built here when
-    /root/reference is present; on the GPU box the prebuilt oracle/_ref/ travels with the snapshot)."""
+    """The reference's own shader source of one pass, compiled for the CPU by oracle/build_refshaders.py (only where the reference
+    sources are present; used to record tests/golden/reference_shader_outputs.npz.xz)."""
     path = reference_shader_path(shader_file_name)
     if path not in _REFSHADERS:
         lib = C.CDLL(path)
@@ -137,8 +208,8 @@ class CpuDenoiser(object):
                 ox, oy = rect_origin if name in harness.RECT_ORIGIN_INPUTS else (0, 0)
                 arr[oy:oy + src.shape[0], ox:ox + src.shape[1]] = src
 
-    def run_dispatch(self, d):
-        lib = self.lib
+    def run_dispatch(self, d, lib=None):
+        lib = lib or self.lib
         texs = (OracleTexture * len(d.resources))()
         keep = []
         from raytracingdenoiser_b200 import harness
@@ -176,15 +247,55 @@ class CpuDenoiser(object):
             texs[i].firstRow = 0
         return texs, keep
 
+    def _state_key(self, d):
+        h = hashlib.sha1(d.shaderFileName.encode() + bytes(d.constants))
+        h.update(np.array([d.gridWidth, d.gridHeight, self.rect_origin[0], self.rect_origin[1]], dtype=np.int64).tobytes())
+        for _, rtype, index in d.resources:
+            arr, fmt = self.resolve(rtype, index)
+            h.update(np.array((int(rtype), int(fmt)) + arr.shape, dtype=np.int64).tobytes())
+            h.update(np.ascontiguousarray(arr).tobytes())
+        return h.digest()[:8]
+
     def run_reference_shader(self, d):
-        """Executes the dispatch with the REFERENCE's own shader source compiled for the CPU (oracle/build_refshaders.py ->
-        oracle/_ref/shaders/<shader>.so) instead of the oracle's restatement of it."""
-        lib = reference_shader_lib(d.shaderFileName)
-        texs, keep = self._textures(d)
-        buf = C.create_string_buffer(d.constants, (len(d.constants) + 15) // 16 * 16)
-        r = lib.refshader_dispatch(buf, len(d.constants), texs, len(d.resources), d.gridWidth, d.gridHeight)
-        if r != 0:
-            raise RuntimeError("refshader_dispatch(%s) failed with %d" % (d.shaderFileName, r))
+        """Executes the dispatch as the REFERENCE's own shader source compiled for the CPU (oracle/build_refshaders.py) computes it:
+        replayed from tests/golden/reference_shader_outputs.npz.xz, or -- in RECORD_ENV mode -- run from oracle/_ref/shaders/<shader>.so
+        and recorded."""
+        outs = [self.resolve(rtype, index)[0] for dtype, rtype, index in d.resources if dtype == nrd.DescriptorType.STORAGE_TEXTURE]
+        key = self._state_key(d)
+        if _recording():
+            before = [a.copy() for a in outs]
+            self.run_dispatch(d, oracle_lib())
+            mine = [a.copy() for a in outs]
+            for a, b in zip(outs, before):
+                a[...] = b
+            lib = reference_shader_lib(d.shaderFileName)
+            texs, keep = self._textures(d)
+            buf = C.create_string_buffer(d.constants, (len(d.constants) + 15) // 16 * 16)
+            r = lib.refshader_dispatch(buf, len(d.constants), texs, len(d.resources), d.gridWidth, d.gridHeight)
+            if r != 0:
+                raise RuntimeError("refshader_dispatch(%s) failed with %d" % (d.shaderFileName, r))
+            record = []
+            for a, m in zip(outs, mine):
+                t, tm = _texels(a), _texels(m)
+                idx = np.nonzero((t != tm).any(axis=1))[0].astype(np.int32)
+                record.append((_digest(a), idx, t[idx] ^ tm[idx]))
+            _recorded[key] = record
+            return
+        g = _golden_records()
+        i = g["index"].get(key)
+        if i is None:
+            raise RuntimeError("%s: no recorded reference-shader output for this input state (inputs, scheduler or an earlier oracle pass changed "
+                               "since tests/golden/reference_shader_outputs.npz.xz was recorded)" % d.shaderFileName)
+        self.run_dispatch(d, oracle_lib())
+        first, last = g["out_start"][i], g["out_start"][i + 1]
+        assert last - first == len(outs), (d.shaderFileName, last - first, len(outs))
+        for a, o in zip(outs, range(first, last)):
+            t = _texels(a)
+            idx = np.cumsum(g["diff_index"][g["diff_start"][o]:g["diff_start"][o + 1]])
+            t[idx] ^= g["diff_value"][g["value_start"][o]:g["value_start"][o + 1]].reshape(t.shape[1], len(idx)).T
+            if _digest(a) != g["out_sha"][o].tobytes():
+                raise RuntimeError("%s: the oracle's output changed since tests/golden/reference_shader_outputs.npz.xz was recorded; the "
+                                   "reference shader's output cannot be reproduced from it" % d.shaderFileName)
 
     def run_both(self, d):
         """Runs the dispatch twice on the same state -- the oracle's pass, then the reference's own shader -- and returns

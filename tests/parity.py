@@ -78,8 +78,7 @@ class SideBySide(object):
         self.report = []
 
     def _cpu_run(self, d):
-        import os
-        if self.reference_shaders and os.path.exists(orr.reference_shader_path(d.shaderFileName)):
+        if self.reference_shaders and orr.has_reference_shader(d.shaderFileName):
             self.cpu.run_reference_shader(d)
         else:
             self.cpu.run_dispatch(d)

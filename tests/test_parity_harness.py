@@ -2,9 +2,6 @@
 instance with its own textures behind the executor's upload / download / execute_raw interface -- takes the place of
 nrd.CudaContext.  Checks the harness logic the GPU tests rely on (state synchronisation before every pass, output comparison, the
 reference-shader mode of tests/test_zz_gpu_reference_shaders.py) on every CPU run."""
-import os
-
-import numpy as np
 import pytest
 
 import oracle_runner as orr
@@ -42,7 +39,6 @@ def test_harness_detects_a_different_evaluation():
     assert any(r["worst"] > 0.0 for r in report) and min(r["fraction"] for r in report) > 0.98
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "shaders")), reason="needs oracle/_ref/shaders")
 @pytest.mark.parametrize("denoiser_name,gate", [("REBLUR_DIFFUSE_SPECULAR", 0.995), ("SIGMA_SHADOW", 0.995), ("RELAX_DIFFUSE_SPECULAR", 0.98)])
 def test_reference_shader_mode_of_the_harness(denoiser_name, gate):
     """tests/test_zz_gpu_reference_shaders.py with the oracle in the role of the kernels: same call, same gates."""

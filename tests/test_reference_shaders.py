@@ -1,6 +1,7 @@
 """The oracle against the code it restates: the reference's OWN pass shaders (/root/reference/Shaders/Source/*.cs.hlsl), compiled for
 the CPU by oracle/build_refshaders.py, are run on exactly the state the oracle's pass is run on, dispatch by dispatch, and every
-texture the pass writes is compared.
+texture the pass writes is compared.  The shaders' outputs are replayed, exactly, from tests/golden/reference_shader_outputs.npz.xz
+(recorded by tests/golden/make_reference_golden.py where the reference sources are present; see tests/oracle_runner.py).
 
 What is the reference in these runs: every statement of the pass body and of Common.hlsli / REBLUR_Common.hlsli / RELAX_Common.hlsli /
 SIGMA_Common.hlsli / NRD.hlsli / Poisson.hlsli, the resource lists, the group sizes, the groupshared preloads and barriers.
@@ -31,8 +32,6 @@ Two deviations of the oracle (and therefore of the kernels, which are held to th
     to a nearest sampler), the shader source evaluates uv first.  With a checkerboarded input, frame 0 (identity rotator) and the
     minimum blur radius of exactly one pixel, offsets of -0.5 land EXACTLY on a texel border and the two evaluations pick
     different neighbours for 27 of 6144 pixels; the pre-pass of that case is held to >= 99.5 % instead of bit-identity."""
-import os
-
 import numpy as np
 import pytest
 
@@ -43,13 +42,6 @@ W, H = 96, 64
 ROUNDING_SENSITIVE = ("RELAX_DiffuseSpecular_TemporalAccumulation", "RELAX_Specular_TemporalAccumulation", "RELAX_Diffuse_TemporalAccumulation",
                       "REBLUR_DiffuseSpecular_TemporalAccumulation", "REBLUR_Specular_TemporalAccumulation", "REBLUR_Perf_DiffuseSpecular_TemporalAccumulation",
                       "_HistoryFix", "_Atrous", "_AntiFirefly")
-
-
-def _have_shaders():
-    return os.path.isdir(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "shaders"))
-
-
-pytestmark = pytest.mark.skipif(not _have_shaders(), reason="oracle/_ref/shaders is built from /root/reference (not present here)")
 
 
 def _checkerboard(mode):
@@ -106,7 +98,7 @@ def run_case(name, variant="", size=None):
         cpu.rect_origin = (0, 0)
         cpu.instance.set_common_settings(harness.make_common_settings(fr, W, H, f, common=common))
         for d in cpu.instance.get_compute_dispatches([cpu.identifier]):
-            if not os.path.exists(orr.reference_shader_path(d.shaderFileName)):
+            if not orr.has_reference_shader(d.shaderFileName):
                 missing.add(d.shaderFileName)
                 cpu.run_dispatch(d)
                 continue
@@ -196,7 +188,7 @@ def test_oracle_chain_against_the_reference_shader_chain(den_name, variant, gate
             cpu.rect_origin = (0, 0)
             cpu.instance.set_common_settings(cs)
             for d in cpu.instance.get_compute_dispatches([cpu.identifier]):
-                if use_ref and os.path.exists(orr.reference_shader_path(d.shaderFileName)):
+                if use_ref and orr.has_reference_shader(d.shaderFileName):
                     cpu.run_reference_shader(d)
                 else:
                     cpu.run_dispatch(d)
